@@ -7,6 +7,9 @@ line from rank 0.  Metric/config = BASELINE.json: GPT-2 (examples/GPT2/345M.json
 synthetic `fake_input` tokens, random-init weights.  Every step = forward + backward + gradient sync +
 optimizer update.  `--impl reference` is the reference arm (see DESIGN.md: the TensorFlow-fork reference
 cannot be installed offline, so it reports `unavailable`).
+
+Tokens and initial weights are seeded, so runs with the same arguments start from identical inputs; `--dump-outputs DIR`
+writes what the last timed step computed, so that two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -19,6 +22,9 @@ import threading
 import time
 
 REF_BASELINE_TOKENS_PER_S = None  # BASELINE.md: the reference publishes no number
+
+# the benchmark may run from a read-only tree: leave it as the build left it
+sys.dont_write_bytecode = True
 
 
 def clocks_sampler(stop_evt, samples, gpu_index):
@@ -67,7 +73,11 @@ def main():
     ap.add_argument("--no-tp", action="store_true", help="skip the tensor-parallel arm (N > 1)")
     ap.add_argument("--no-library-arm", action="store_true",
                     help="skip the same-box library comparator (cuBLAS / SDPA / per-tensor NCCL step, bench/torch_baseline.py)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (its loss, rank 0) as DIR/loss.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     if args.impl == "reference":
         print(json.dumps({"impl": "reference", "unavailable":
@@ -159,6 +169,13 @@ def main():
     ms = e0.elapsed_time(e1)
     launches = ops.launch_count()
     final_loss = float(loss)
+    if args.dump_outputs and rank == 0:
+        # The step returns the loss and nothing else.  The weights it updates are not dumped: the gradient reductions add
+        # with float atomics, and AdamW turns gradients at noise level (the attention key bias's is exactly zero) into
+        # full-size updates, so the weights differ from run to run by far more than the loss does.
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "loss.npy"), loss.detach().float().reshape(-1).cpu().numpy())
 
     # ---------------- end-to-end through the public API: H2D inputs from pinned memory + D2H loss every step
     barrier()
@@ -301,6 +318,8 @@ def main():
             "final_loss": final_loss,
             "clocks": summarize_clocks(samples),
         }
+        if args.dump_outputs:
+            out["dump_outputs"] = {"dir": args.dump_outputs, "arrays": ["loss"]}
         if ms_lib > 0:
             out["library_arm"] = {"ms_per_step": ms_lib / K, "tokens_per_s": tokens / (ms_lib / 1e3), "ours_over_library": ms_lib / ms,
                                   "what": "same box, same process: torch cuBLAS / SDPA / fused AdamW + per-tensor in-stream NCCL all-reduce, CUDA graph"}
