@@ -30,11 +30,14 @@ def main():
     ap.add_argument("--data", default=None, help="comma-separated token files (see tepdist_b200.data.write_token_file) or 'synthetic'")
     ap.add_argument("--data-int32", action="store_true", help="token files hold int32 ids (default uint16)")
     ap.add_argument("--seed", type=int, default=0)
+    ap.add_argument("--doc-mask", action="store_true",
+                    help="document masking: attention stays inside each document of a packed window (documents end at --eot)")
+    ap.add_argument("--eot", type=int, default=50256, help="end-of-text token id that closes a document (GPT-2 BPE: 50256)")
     a = ap.parse_args()
     clip = {"clip_norm": a.clip_norm, "clip_norm_value": a.clip_norm_value} if a.clip_norm else {}
     cfg = CONFIGS[a.model]
     world = int(os.environ.get("WORLD_SIZE", "1"))
-    g = build_gpt2_graph(cfg, batch=a.batch * world, optimizer=a.optimizer, **clip)
+    g = build_gpt2_graph(cfg, batch=a.batch * world, optimizer=a.optimizer, doc_mask=a.doc_mask, **clip)
     tr = Trainer(g, strategy=a.strategy, comm_mode=a.comm)
     if a.warmup_steps > 0:
         from tepdist_b200.utils.schedules import warmup_cosine
@@ -44,11 +47,14 @@ def main():
         # columns its plan assigns to this rank: works unchanged under data, tensor, context and pipeline parallel plans
         from tepdist_b200.data import TokenLoader
         src = {"synthetic_vocab": cfg.n_vocab} if a.data == "synthetic" else {"files": a.data.split(","), "bytes_per_token": 4 if a.data_int32 else 2}
-        batches = iter(TokenLoader(batch=a.batch * world, n_ctx=cfg.n_ctx, seed=a.seed, **src))
+        batches = iter(TokenLoader(batch=a.batch * world, n_ctx=cfg.n_ctx, seed=a.seed, eot=a.eot if a.doc_mask else None, **src))
     else:
         gen = torch.Generator().manual_seed(a.seed)
         tok = torch.randint(0, cfg.n_vocab, (a.batch * world, cfg.n_ctx), generator=gen, dtype=torch.int32)
         fixed = {"tokens": tok, "labels": torch.roll(tok, -1, 1)}
+        if a.doc_mask:
+            from tepdist_b200.data import segments_from_tokens
+            fixed["segments"] = segments_from_tokens(tok, a.eot)
         batches = iter(lambda: fixed, None)
     t0 = time.time()
     for i in range(a.train_steps):

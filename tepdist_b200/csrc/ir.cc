@@ -213,6 +213,7 @@ double NodeFlops(const Graph& g, const Node& n) {
     else { w = &n.outputs[0]; y = &g.type(n.inputs[0]); }
     return 2.0 * (double)y->numel() * (double)(w->dims[1] * w->dims[2] * w->dims[3]);
   }
+  // Attention FLOPs stay the causal / full count with document masking too: document lengths are only known from the data.
   if (op == "attention") {
     const TensorType& qkv = g.type(n.inputs[0]);
     double B = qkv.dims[0], S = qkv.dims[1], C = qkv.dims[2] / 3.0;

@@ -205,21 +205,26 @@ void LayerNormBwdRule(Ctx& c) {
 // merge by log-sum-exp.  The reference has no such op (SURVEY 5.7: long context = token split + what XLA SPMD makes of the dots);
 // priced as the K / V all-gather it replaces (forward) plus the dK / dV reduce-scatter (backward).
 double RingBytes(const TensorType& qkv, int num) { return (double)qkv.bytes() * (2.0 / 3.0) * (num - 1) / num; }
+// Optional document ids (int32 [B, S], the last input; no gradient): they follow qkv's batch split and stay whole along the
+// sequence in "seq", so every rank of the ring already holds the key ids of every visiting block and the ring carries no extra
+// bytes (ids cost 4 bytes a token against 4 C for the K / V block).  Replicated in "heads" and "glue".
 void AttentionRule(Ctx& c, const RuleOptions& opt) {
-  // qkv [B,S,H*3*D] (heads-major, so a plain last-dim split is a split over heads) -> o [B,S,H*D], lse [B,H,S]
+  // qkv [B,S,H*3*D] (heads-major, so a plain last-dim split is a split over heads) [, segments [B,S]] -> o [B,S,H*D], lse [B,H,S]
   const int64_t H = c.n.attr_i("heads");
   const bool cp = opt.context_parallel && c.divisible(c.in(0), 1);   // "cp": the sequence split is the only way through attention
-  if (c.divisible(c.in(0), 0) && !cp) c.add({c.S(0)}, {c.S(0), c.S(0)}, "batch");
-  if (H % c.num == 0 && !cp) c.add({c.S(2)}, {c.S(2), c.S(1)}, "heads");
-  if (c.divisible(c.in(0), 1)) c.add({c.S(1)}, {c.S(1), c.S(2)}, "seq", RingBytes(c.in(0), c.num));
+  auto ins = [&](DS qkv, DS seg) { return c.nin() > 1 ? std::vector<DS>{qkv, seg} : std::vector<DS>{qkv}; };
+  if (c.divisible(c.in(0), 0) && !cp) c.add(ins(c.S(0), c.S(0)), {c.S(0), c.S(0)}, "batch");
+  if (H % c.num == 0 && !cp) c.add(ins(c.S(2), c.G()), {c.S(2), c.S(1)}, "heads");
+  if (c.divisible(c.in(0), 1)) c.add(ins(c.S(1), c.G()), {c.S(1), c.S(2)}, "seq", RingBytes(c.in(0), c.num));
   if (!cp) c.add_glue();   // (replicated attention = n x the S^2 FLOPs per rank: never what "cp" asks for)
 }
 void AttentionBwdRule(Ctx& c, const RuleOptions& opt) {
-  const int64_t H = c.n.attr_i("heads");  // (do, qkv, o, lse) -> dqkv
+  const int64_t H = c.n.attr_i("heads");  // (do, qkv, o, lse [, segments]) -> dqkv
   const bool cp = opt.context_parallel && c.divisible(c.in(1), 1);
-  if (c.divisible(c.in(1), 0) && !cp) c.add({c.S(0), c.S(0), c.S(0), c.S(0)}, {c.S(0)}, "batch");
-  if (H % c.num == 0 && !cp) c.add({c.S(2), c.S(2), c.S(2), c.S(1)}, {c.S(2)}, "heads");
-  if (c.divisible(c.in(1), 1)) c.add({c.S(1), c.S(1), c.S(1), c.S(2)}, {c.S(1)}, "seq", 2.0 * RingBytes(c.in(1), c.num));
+  auto ins = [&](std::vector<DS> v, DS seg) { if (c.nin() > 4) v.push_back(seg); return v; };
+  if (c.divisible(c.in(1), 0) && !cp) c.add(ins({c.S(0), c.S(0), c.S(0), c.S(0)}, c.S(0)), {c.S(0)}, "batch");
+  if (H % c.num == 0 && !cp) c.add(ins({c.S(2), c.S(2), c.S(2), c.S(1)}, c.G()), {c.S(2)}, "heads");
+  if (c.divisible(c.in(1), 1)) c.add(ins({c.S(1), c.S(1), c.S(1), c.S(2)}, c.G()), {c.S(1)}, "seq", 2.0 * RingBytes(c.in(1), c.num));
   if (!cp) c.add_glue();
 }
 void EmbeddingRule(Ctx& c) {  // tokens[B,S], wte[V,C], wpe[S,C] -> [B,S,C]

@@ -119,13 +119,18 @@ BatchLoader::BatchLoader(std::shared_ptr<TokenSource> src, int batch, int n_ctx,
 }
 BatchLoader::~BatchLoader() { Stop(); }
 
-void BatchLoader::SetBuffers(const std::vector<uintptr_t>& tokens, const std::vector<uintptr_t>& labels) {
+void BatchLoader::SetBuffers(const std::vector<uintptr_t>& tokens, const std::vector<uintptr_t>& labels,
+                             const std::vector<uintptr_t>& segments, int32_t eot) {
   if (running_) throw std::runtime_error("SetBuffers while running");
   if (tokens.empty() || tokens.size() != labels.size()) throw std::invalid_argument("need one tokens and one labels buffer per slot");
+  if (!segments.empty() && segments.size() != tokens.size()) throw std::invalid_argument("need one segments buffer per slot, or none");
   tok_.clear();
   lab_.clear();
+  seg_.clear();
   for (auto p : tokens) tok_.push_back(reinterpret_cast<int32_t*>(p));
   for (auto p : labels) lab_.push_back(reinterpret_cast<int32_t*>(p));
+  for (auto p : segments) seg_.push_back(reinterpret_cast<int32_t*>(p));
+  eot_ = eot;
   state_.assign(tok_.size(), kFree);
   slot_step_.assign(tok_.size(), 0);
 }
@@ -162,6 +167,14 @@ void BatchLoader::Fill(int slot, uint64_t step) {
     src_->Sample(seed_, sample, n, win.data());
     std::memcpy(tok_[slot] + (size_t)b * n_ctx_, win.data(), sizeof(int32_t) * (size_t)n_ctx_);
     std::memcpy(lab_[slot] + (size_t)b * n_ctx_, win.data() + 1, sizeof(int32_t) * (size_t)n_ctx_);   // next-token labels
+    if (!seg_.empty()) {
+      int32_t* seg = seg_[slot] + (size_t)b * n_ctx_;
+      int32_t d = 0;
+      for (int i = 0; i < n_ctx_; ++i) {
+        seg[i] = d;
+        d += win[(size_t)i] == eot_;
+      }
+    }
   }
 }
 

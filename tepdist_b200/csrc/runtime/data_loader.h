@@ -68,8 +68,11 @@ class BatchLoader {
  public:
   BatchLoader(std::shared_ptr<TokenSource> src, int batch, int n_ctx, int rank, int world, uint64_t seed, int threads);
   ~BatchLoader();
-  // slot buffers: int32 [batch, n_ctx] each, owned by the caller (torch pinned tensors) and alive until Stop()
-  void SetBuffers(const std::vector<uintptr_t>& tokens, const std::vector<uintptr_t>& labels);
+  // slot buffers: int32 [batch, n_ctx] each, owned by the caller (torch pinned tensors) and alive until Stop().
+  // Optional `segments` buffers (one per slot, or none) receive document ids: seg[i] = number of `eot` tokens at window
+  // positions < i, so the end-of-text token belongs to the document it ends.
+  void SetBuffers(const std::vector<uintptr_t>& tokens, const std::vector<uintptr_t>& labels,
+                  const std::vector<uintptr_t>& segments = {}, int32_t eot = 0);
   void Start(uint64_t first_step);
   // Blocks until the batch of the next step is complete; returns its slot.  Steps are handed out in order.
   int Acquire(uint64_t* step);
@@ -85,7 +88,8 @@ class BatchLoader {
   std::shared_ptr<TokenSource> src_;
   int batch_, n_ctx_, rank_, world_, threads_;
   uint64_t seed_;
-  std::vector<int32_t*> tok_, lab_;
+  std::vector<int32_t*> tok_, lab_, seg_;
+  int32_t eot_ = 0;
   // slot state machine: kFree -> (claimed by a worker for step s) kFilling -> kReady -> (Acquire) kInUse -> (Release) kFree
   enum State { kFree, kFilling, kReady, kInUse };
   std::vector<State> state_;

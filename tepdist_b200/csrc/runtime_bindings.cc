@@ -33,7 +33,8 @@ void BindRuntime(py::module_& m) {
   py::class_<BatchLoader>(m, "BatchLoader")
       .def(py::init<std::shared_ptr<TokenSource>, int, int, int, int, uint64_t, int>(), py::arg("source"), py::arg("batch"), py::arg("n_ctx"),
            py::arg("rank") = 0, py::arg("world") = 1, py::arg("seed") = 0, py::arg("threads") = 2)
-      .def("set_buffers", &BatchLoader::SetBuffers)
+      .def("set_buffers", &BatchLoader::SetBuffers, py::arg("tokens"), py::arg("labels"),
+           py::arg("segments") = std::vector<uintptr_t>{}, py::arg("eot") = 0)
       .def("start", &BatchLoader::Start, py::arg("first_step") = 0)
       .def("acquire", [](BatchLoader& l) {
         uint64_t step = 0;

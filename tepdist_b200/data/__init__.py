@@ -14,6 +14,8 @@ module offers the same through `_C.TokenSource` / `_C.BatchLoader` (csrc/runtime
 * `prefetch` slots of page-locked memory are filled ahead by `threads` native threads; a yielded batch stays valid until the next
   one is requested (the training step's host->device copy reads straight from it).
 * `mix=[(files, weight), ...]`: several datasets sampled by weight; `synthetic_vocab=V`: random tokens (the reference's fake_input).
+* `eot=50256`: batches also carry "segments", int32 [batch, n_ctx] document ids for document-masked attention
+  (`build_gpt2_graph(..., doc_mask=True)`), filled by the same native threads: `segments_from_tokens(tokens, eot)`.
 """
 from __future__ import annotations
 
@@ -36,12 +38,21 @@ def write_token_file(path: str, tokens, dtype: str = "auto") -> Tuple[str, int]:
     return path, 2 if dtype == "uint16" else 4
 
 
+def segments_from_tokens(tokens: torch.Tensor, eot: int) -> torch.Tensor:
+    """Document ids of packed windows [..., n]: seg[i] = number of `eot` tokens at positions < i along the last dim, so the
+    end-of-text token belongs to the document it ends.  int32, on the device of `tokens` (CPU or CUDA)."""
+    ends = (tokens == eot).to(torch.int32)
+    seg = torch.cumsum(ends, -1, dtype=torch.int32) - ends
+    return seg
+
+
 class TokenLoader:
     """Iterator over this rank's batches; see the module docstring."""
 
     def __init__(self, files: Optional[Files] = None, *, batch: int, n_ctx: int, rank: int = 0, world: int = 1, seed: int = 0,
                  mix: Optional[Sequence[Tuple[Files, float]]] = None, synthetic_vocab: int = 0, bytes_per_token: int = 2,
-                 prefetch: int = 4, threads: int = 2, start_step: int = 0, steps: Optional[int] = None, pin: Optional[bool] = None):
+                 prefetch: int = 4, threads: int = 2, start_step: int = 0, steps: Optional[int] = None, pin: Optional[bool] = None,
+                 eot: Optional[int] = None):
         from .. import _C
         if sum(x is not None and x != 0 for x in (files, mix, synthetic_vocab)) != 1:
             raise ValueError("give exactly one of files=, mix= or synthetic_vocab=")
@@ -58,7 +69,10 @@ class TokenLoader:
         self._tok: List[torch.Tensor] = [mk() for _ in range(max(2, int(prefetch)))]
         self._lab: List[torch.Tensor] = [mk() for _ in range(len(self._tok))]
         self._loader = _C.BatchLoader(self.source, self.batch, self.n_ctx, self.rank, self.world, self.seed, int(threads))
-        self._loader.set_buffers([t.data_ptr() for t in self._tok], [t.data_ptr() for t in self._lab])
+        self.eot = None if eot is None else int(eot)
+        self._seg: List[torch.Tensor] = [mk() for _ in range(len(self._tok))] if self.eot is not None else []
+        self._loader.set_buffers([t.data_ptr() for t in self._tok], [t.data_ptr() for t in self._lab],
+                                 [t.data_ptr() for t in self._seg], 0 if self.eot is None else self.eot)
         self._held: Optional[int] = None
         self.step = int(start_step)          # step of the NEXT batch
         self._first = int(start_step)
@@ -77,6 +91,8 @@ class TokenLoader:
         assert step == self.step, (step, self.step)
         self._held = slot
         self.step += 1
+        if self.eot is not None:
+            return {"tokens": self._tok[slot], "labels": self._lab[slot], "segments": self._seg[slot]}
         return {"tokens": self._tok[slot], "labels": self._lab[slot]}
 
     def close(self) -> None:

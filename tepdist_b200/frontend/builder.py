@@ -82,10 +82,16 @@ class GraphBuilder:
     def gelu(self, x: Value, name="gelu") -> Value:
         return self._n("gelu", [x], [self.t(x)], {}, name).out()
 
-    def attention(self, qkv: Value, heads: int, causal: bool = True, name="attn") -> Value:
+    def attention(self, qkv: Value, heads: int, causal: bool = True, segments: Optional[Value] = None, name="attn") -> Value:
+        """Fused attention over qkv [B, S, 3C].  `segments` (int32 [B, S], optional): document ids; query i attends to key j
+        only if segments[i] == segments[j] (and j <= i when causal)."""
         B, S, C3 = self.t(qkv).shape
         C = C3 // 3
-        n = self._n("attention", [qkv], [TensorType((B, S, C), self.t(qkv).dtype), TensorType((B, heads, S), "f32")],
+        ins = [qkv]
+        if segments is not None:
+            assert tuple(self.t(segments).shape) == (B, S) and self.t(segments).dtype == "i32", self.t(segments)
+            ins.append(segments)
+        n = self._n("attention", ins, [TensorType((B, S, C), self.t(qkv).dtype), TensorType((B, heads, S), "f32")],
                     {"heads": heads, "causal": causal}, name)
         return n.out(0)
 
@@ -344,7 +350,8 @@ def backward(b: GraphBuilder, loss: Value) -> Dict[int, Value]:
             push(n.inputs[0], B("gelu_bwd", [dy, n.inputs[0]], [T(n.inputs[0])], {}, grp).out())
         elif n.op == "attention":
             qkv = n.inputs[0]
-            push(qkv, B("attention_bwd", [dy, qkv, Value(n.id, 0), Value(n.id, 1)], [T(qkv)], dict(n.attrs), grp).out())
+            push(qkv, B("attention_bwd", [dy, qkv, Value(n.id, 0), Value(n.id, 1)] + list(n.inputs[1:]), [T(qkv)], dict(n.attrs),
+                        grp).out())
         elif n.op == "embedding":
             tok, wte, wpe = n.inputs
             nb = B("embedding_bwd", [tok, dy], [TensorType(T(wte).shape, "f32"), TensorType(T(wpe).shape, "f32")], {}, grp)

@@ -51,12 +51,16 @@ CONFIGS = {
 }
 
 
-def build_gpt2_graph(cfg: GPT2Config, batch: int | None = None, optimizer: str = "adamw", **opt_hp) -> Graph:
+def build_gpt2_graph(cfg: GPT2Config, batch: int | None = None, optimizer: str = "adamw", doc_mask: bool = False,
+                     **opt_hp) -> Graph:
+    """`doc_mask=True`: a third input "segments" (int32 [B, n_ctx] document ids, e.g. `TokenLoader(..., eot=50256)` or
+    `data.segments_from_tokens`) keeps every layer's attention inside each packed document."""
     B = batch or cfg.batch
     S, C, H, V, Vp = cfg.n_ctx, cfg.n_embd, cfg.n_head, cfg.n_vocab, cfg.padded_vocab
     b = GraphBuilder(cfg.name)
     tokens = b.input("tokens", (B, S), "i32")
     labels = b.input("labels", (B, S), "i32")
+    segments = b.input("segments", (B, S), "i32") if doc_mask else None
     nrm = lambda std: {"kind": "normal", "mean": 0.0, "std": std}
     const = lambda v: {"kind": "constant", "value": v}
     with b.scope("model"):
@@ -69,7 +73,7 @@ def build_gpt2_graph(cfg: GPT2Config, batch: int | None = None, optimizer: str =
                 h = b.layernorm(x, g1, b1, name="ln_1")
                 w_qkv = b.parameter("attn/c_attn/w", (3 * C, C), nrm(0.02)); b_qkv = b.parameter("attn/c_attn/b", (3 * C,), const(0.0))
                 qkv = b.linear(h, w_qkv, b_qkv, name="attn/c_attn")
-                a = b.attention(qkv, heads=H, causal=True, name="attn/core")
+                a = b.attention(qkv, heads=H, causal=True, segments=segments, name="attn/core")
                 w_o = b.parameter("attn/c_proj/w", (C, C), nrm(0.02 / math.sqrt(2 * cfg.n_layer))); b_o = b.parameter("attn/c_proj/b", (C,), const(0.0))
                 x = b.linear(a, w_o, b_o, residual=x, name="attn/c_proj")
                 g2 = b.parameter("ln_2/g", (C,), const(1.0)); b2 = b.parameter("ln_2/b", (C,), const(0.0))
@@ -87,5 +91,5 @@ def build_gpt2_graph(cfg: GPT2Config, batch: int | None = None, optimizer: str =
     g = build_training_step(b, loss, optimizer, **{**dict(lr=cfg.lr, beta1=0.9, beta2=0.999, eps=1e-8, weight_decay=cfg.weight_decay),
                                                      **opt_hp})      # (opt_hp: clip_norm / clip_norm_value / schedule / ...)
     g.meta["model"] = {"family": "gpt2", "name": cfg.name, "n_layer": cfg.n_layer, "n_embd": C, "n_head": H,
-                       "n_ctx": S, "n_vocab": V, "batch": B}
+                       "n_ctx": S, "n_vocab": V, "batch": B, "doc_mask": bool(doc_mask)}
     return g

@@ -107,9 +107,9 @@ class _Sig:
     tepd_gap_bwd_nhwc = [_vp, _vp, _i, _i, _i, _vp]
     tepd_attn_merge = [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]
     tepd_attn_ring_accum = [_vp, _vp, _vp, _ll, _i, _i, _vp]
-    tepd_attn_fwd = [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _f, _i, _ll, _ll, _ll, _vp]
+    tepd_attn_fwd = [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _f, _i, _ll, _ll, _ll, _vp, _vp, _ll, _vp]
     tepd_attn_bwd = [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _f, _i,
-                     _ll, _ll, _ll, _ll, _ll, _ll, _vp]
+                     _ll, _ll, _ll, _ll, _ll, _ll, _vp, _vp, _ll, _vp]
 
 
 def _stream() -> int:

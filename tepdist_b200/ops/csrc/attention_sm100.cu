@@ -36,6 +36,7 @@ constexpr int HD = 64;        // head dim
 constexpr int BQ = 128;       // query rows per CTA
 constexpr int BKV = 128;      // kv rows per iteration
 constexpr int KV_STAGES = 3;
+constexpr int SEG_MAX_BLOCKS = 2048;   // S <= 262144: the visited-block list lives in shared memory
 constexpr int FWD_THREADS = 64 + 256;
 
 constexpr int TILE_BYTES = 128 * HD * 2;  // 16 KB: a [128 x 64] bf16 tile (one SW128 chunk)
@@ -46,6 +47,60 @@ constexpr int SM_P = SM_V + KV_STAGES * TILE_BYTES;   // [128 x 128] bf16 = 2 ch
 constexpr int SM_BAR = SM_P + 2 * TILE_BYTES;
 constexpr int SM_MAX = SM_BAR + 256;                  // float [2 iter parity][2 halves][128]
 constexpr int FWD_SMEM = SM_MAX + 2 * 2 * 128 * 4 + 1024;
+constexpr int SM_SEG_IDS = SM_MAX + 2 * 2 * 128 * 4;              // SEG: int [KV_STAGES][128] key ids
+constexpr int SM_SEG_LIST = SM_SEG_IDS + KV_STAGES * 128 * 4;     // SEG: int visited count, then the list
+constexpr int FWD_SEG_SMEM = SM_SEG_LIST + 16 + SEG_MAX_BLOCKS * 4 + 1024;
+
+// Document masking (SEG = 1 instantiations).  Query i may attend to key j only if seg_q[i] == seg_k[j] (on top of the causal
+// rule).  attn_seg_range_kernel first writes the [min, max] id of every 128-row block; a (query block, key block) pair whose
+// intervals do not overlap is skipped, and inside a visited block the 128 key ids staged in shared memory next to K / V mask
+// element-wise (skipped for rows whose document covers the whole key block).  Skipping is an optimisation only: any int32 ids
+// give exact results.  Rows that see no key at all produce o = 0, lse = -inf.
+struct AttnSeg {
+  const int* seg_q;     // int32, row b at seg_q + b * stride
+  const int* seg_k;
+  const int2* rng_q;    // [B, S / 128] (min, max) of the query ids of each block
+  const int2* rng_k;
+  long long stride;
+};
+
+__device__ __forceinline__ bool seg_overlap(int2 a, int2 b) { return a.x <= b.y && b.x <= a.y; }
+
+// 1-D bulk copy global -> shared, completing on an mbarrier (16-byte aligned, size a multiple of 16)
+__device__ __forceinline__ void bulk_load(void* smem_dst, const void* src, uint32_t bytes, uint64_t* bar) {
+  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+               ::"r"(smem_u32(smem_dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
+}
+
+// One warp per (batch row, 128-id block): out[b * nblk + blk] = (min, max).  blockIdx.y selects the query (0) or key (1) ids.
+__global__ void __launch_bounds__(256) attn_seg_range_kernel(const AttnSeg sg, int2* rng_q, int2* rng_k, int B, int nblk) {
+  const int w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+  pdl_wait();
+  if (w >= B * nblk) return;
+  const int b = w / nblk, blk = w % nblk;
+  const int* src = (blockIdx.y ? sg.seg_k : sg.seg_q) + b * sg.stride + blk * 128;
+  const int4 x = reinterpret_cast<const int4*>(src)[lane];
+  int mn = min(min(x.x, x.y), min(x.z, x.w)), mx = max(max(x.x, x.y), max(x.z, x.w));
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    mn = min(mn, __shfl_xor_sync(0xffffffffu, mn, o));
+    mx = max(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+  }
+  if (lane == 0) (blockIdx.y ? rng_k : rng_q)[w] = make_int2(mn, mx);
+}
+
+// Visited-block list of one CTA, built by one warp: list[k] = the k-th block c in [c0, c1) with seg_overlap(mine, rng[c]).
+__device__ __forceinline__ int seg_visit_list(const int2* rng, int c0, int c1, int2 mine, int* list, int lane) {
+  int n = 0;
+  for (int base = c0; base < c1; base += 32) {
+    const int c = base + lane;
+    const bool vis = c < c1 && seg_overlap(mine, rng[c]);
+    const unsigned m = __ballot_sync(0xffffffffu, vis);
+    if (vis) list[n + __popc(m & ((1u << lane) - 1u))] = c;
+    n += __popc(m);
+  }
+  return n;
+}
 
 struct AttnFwdParams {
   void* O;      // bf16 [B, S, H, D]
@@ -75,10 +130,10 @@ __device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
 
-template <int POLY>
+template <int POLY, int SEG>
 __global__ void __launch_bounds__(FWD_THREADS, 1)
 attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_k,
-                const __grid_constant__ CUtensorMap tmap_v, const AttnFwdParams p) {
+                const __grid_constant__ CUtensorMap tmap_v, const AttnFwdParams p, const AttnSeg sg) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + SM_BAR);
@@ -99,7 +154,9 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
   const int qb = nq - 1 - (int)(blockIdx.x / BH);  // heavy (long) rows first
   const int bh = blockIdx.x % BH;
   const int b = bh / p.H, h = bh % p.H;
-  const int n_kv = p.causal ? (qb + 1) : (p.S / BKV);
+  int n_kv = p.causal ? (qb + 1) : (p.S / BKV);
+  int* seg_ids = reinterpret_cast<int*>(smem + SM_SEG_IDS);
+  int* seg_list = reinterpret_cast<int*>(smem + SM_SEG_LIST) + 4;
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmap_q);
@@ -123,20 +180,32 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
   const uint32_t tmem_base = *tmem_slot;
   pdl_wait();      // (launch.cuh) the prologue above ran under the previous kernel's tail
   pdl_trigger();
+  if (SEG) {         // every role walks the same list of key blocks whose id interval meets the query block's
+    if (warp == 2) {
+      const int nv = seg_visit_list(sg.rng_k + (size_t)b * nq, 0, n_kv, sg.rng_q[(size_t)b * nq + qb], seg_list, lane);
+      if (lane == 0) seg_list[-1] = nv;
+    }
+    __syncthreads();
+    n_kv = seg_list[-1];
+  }
   const uint32_t TM_S = tmem_base;          // 2 x 128 columns
   const uint32_t TM_PV = tmem_base + 256;   // 64 columns
 
   if (warp == 0) {
     if (elect_one()) {
-      mbar_expect_tx(q_full, TILE_BYTES);
-      tma_load_4d(smem + SM_Q, &tmap_q, q_full, 0, qb * BQ, h, b);
+      if (!SEG || n_kv > 0) {
+        mbar_expect_tx(q_full, TILE_BYTES);
+        tma_load_4d(smem + SM_Q, &tmap_q, q_full, 0, qb * BQ, h, b);
+      }
       for (int j = 0; j < n_kv; ++j) {
         const int st = j % KV_STAGES;
         const uint32_t ph = (j / KV_STAGES) & 1;
+        const int jb = SEG ? seg_list[j] : j;
         mbar_wait(&kv_empty[st], ph ^ 1);
-        mbar_expect_tx(&kv_full[st], 2 * TILE_BYTES);
-        tma_load_4d(smem + SM_K + st * TILE_BYTES, &tmap_k, &kv_full[st], 0, j * BKV, h, b);
-        tma_load_4d(smem + SM_V + st * TILE_BYTES, &tmap_v, &kv_full[st], 0, j * BKV, h, b);
+        mbar_expect_tx(&kv_full[st], 2 * TILE_BYTES + (SEG ? BKV * 4 : 0));
+        tma_load_4d(smem + SM_K + st * TILE_BYTES, &tmap_k, &kv_full[st], 0, jb * BKV, h, b);
+        tma_load_4d(smem + SM_V + st * TILE_BYTES, &tmap_v, &kv_full[st], 0, jb * BKV, h, b);
+        if (SEG) bulk_load(seg_ids + st * BKV, sg.seg_k + b * sg.stride + jb * BKV, BKV * 4, &kv_full[st]);
       }
     }
   } else if (warp == 1) {
@@ -158,8 +227,10 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
         }
         umma_commit(&s_full[j & 1]);
       };
-      mbar_wait(q_full, 0);
-      issue_s(0);
+      if (!SEG || n_kv > 0) {
+        mbar_wait(q_full, 0);
+        issue_s(0);
+      }
       for (int j = 0; j < n_kv; ++j) {
         if (j + 1 < n_kv) issue_s(j + 1);
         mbar_wait(p_full, j & 1);
@@ -187,6 +258,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
     float o[32];
 #pragma unroll
     for (int i = 0; i < 32; ++i) o[i] = 0.f;
+    const int my_seg = SEG ? sg.seg_q[b * sg.stride + q_global] : 0;
 
     for (int j = 0; j < n_kv; ++j) {
       mbar_wait(&s_full[j & 1], (j >> 1) & 1);
@@ -202,10 +274,26 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
       float s[64];
 #pragma unroll
       for (int i = 0; i < 32; ++i) { s[i] = __uint_as_float(r0[i]); s[32 + i] = __uint_as_float(r1[i]); }
-      const int col0 = j * BKV + half * 64;
-      if (p.causal && j == qb) {
+      const int jb = SEG ? seg_list[j] : j;
+      const int col0 = jb * BKV + half * 64;
+      if (p.causal && jb == qb) {
 #pragma unroll
         for (int i = 0; i < 64; ++i) if (col0 + i > q_global) s[i] = -INFINITY;
+      }
+      if (SEG) {
+        const int2 kr = sg.rng_k[(size_t)b * nq + jb];
+        if (!(kr.x == my_seg && kr.y == my_seg)) {   // the key block is not all of this row's document: compare ids
+          mbar_wait(&kv_full[j % KV_STAGES], (j / KV_STAGES) & 1);   // (complete already: S(j) was computed from this stage)
+          const int4* ids = reinterpret_cast<const int4*>(seg_ids + (j % KV_STAGES) * BKV + half * 64);
+#pragma unroll
+          for (int g = 0; g < 16; ++g) {
+            const int4 id = ids[g];
+            if (id.x != my_seg) s[4 * g + 0] = -INFINITY;
+            if (id.y != my_seg) s[4 * g + 1] = -INFINITY;
+            if (id.z != my_seg) s[4 * g + 2] = -INFINITY;
+            if (id.w != my_seg) s[4 * g + 3] = -INFINITY;
+          }
+        }
       }
       float mx = -INFINITY;
 #pragma unroll
@@ -215,8 +303,10 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
       named_bar_sync(1, 256);
       mx = fmaxf(mx, mbuf[(1 - half) * 128 + row]);
       const float m_new = fmaxf(m_run, mx);
-      const float alpha = exp2f((m_run - m_new) * p.scale_log2);  // m_run = -inf -> 0
-      const float mb = m_new * p.scale_log2;
+      // SEG: a row that has seen no key yet keeps m = -inf; a finite stand-in keeps alpha and P at exact zeros instead of NaN
+      const float m_ref = (SEG && m_new == -INFINITY) ? 0.f : m_new;
+      const float alpha = exp2f((m_run - m_ref) * p.scale_log2);  // m_run = -inf -> 0
+      const float mb = m_ref * p.scale_log2;
       float lsum = 0.f;
       uint32_t pk[32];
 #pragma unroll
@@ -256,9 +346,9 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
       if (lane == 0) mbar_arrive(p_full);
     }
     // last P V product
-    mbar_wait(pv_full, (n_kv - 1) & 1);
-    tc_fence_after();
-    {
+    if (!SEG || n_kv > 0) {
+      mbar_wait(pv_full, (n_kv - 1) & 1);
+      tc_fence_after();
       uint32_t pv[32];
       tmem_ld_32x32(TM_PV + lane_addr + half * 32, pv);
       tmem_ld_wait();
@@ -271,7 +361,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
     lbuf[half * 128 + row] = l_run;
     named_bar_sync(1, 256);
     const float l_tot = l_run + lbuf[(1 - half) * 128 + row];
-    const float inv = 1.f / l_tot;
+    const float inv = (SEG && l_tot == 0.f) ? 0.f : 1.f / l_tot;
     __nv_bfloat16* orow = reinterpret_cast<__nv_bfloat16*>(p.O) +
                           (((size_t)b * p.S + q_global) * p.H + h) * HD + half * 32;
 #pragma unroll
@@ -283,7 +373,8 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
       u.w = pack_bf16x2(o[8 * g + 6] * inv, o[8 * g + 7] * inv);
       reinterpret_cast<uint4*>(orow)[g] = u;
     }
-    if (half == 0) p.lse[((size_t)b * p.H + h) * p.S + q_global] = m_run * p.scale + __logf(l_tot);
+    if (half == 0)
+      p.lse[((size_t)b * p.H + h) * p.S + q_global] = (SEG && l_tot == 0.f) ? -INFINITY : m_run * p.scale + __logf(l_tot);
   }
 
   tc_fence_before();
@@ -562,6 +653,9 @@ constexpr int SB_P = SB_DO + 2 * TILE_BYTES;     // 2 chunks
 constexpr int SB_DS = SB_P + 2 * TILE_BYTES;     // 2 chunks
 constexpr int SB_BAR = SB_DS + 2 * TILE_BYTES;
 constexpr int BWD_SMEM = SB_BAR + 256 + 1024;
+constexpr int SB_SEG_IDS = SB_BAR + 256;               // SEG: int [128] key ids of the CTA's kv block
+constexpr int SB_SEG_LIST = SB_SEG_IDS + BKV * 4;      // SEG: int visited count, then the list of query blocks
+constexpr int BWD_SEG_SMEM = SB_SEG_LIST + 16 + SEG_MAX_BLOCKS * 4 + 1024;
 
 struct AttnBwdParams {
   const float* lse;    // [B,H,S]
@@ -574,11 +668,11 @@ struct AttnBwdParams {
   float scale_log2, scale;
 };
 
-template <int POLY>
+template <int POLY, int SEG>
 __global__ void __launch_bounds__(BWD_THREADS, 1)
 attn_bwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_k,
                 const __grid_constant__ CUtensorMap tmap_v, const __grid_constant__ CUtensorMap tmap_do,
-                const AttnBwdParams p) {
+                const AttnBwdParams p, const AttnSeg sg) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + SB_BAR);
@@ -599,7 +693,9 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
   const int bh = blockIdx.x % BH;
   const int b = bh / p.H, h = bh % p.H;
   const int i0 = p.causal ? j : 0;
-  const int n_it = nq - i0;
+  int n_it = nq - i0;
+  int* seg_ids = reinterpret_cast<int*>(smem + SB_SEG_IDS);
+  int* seg_list = reinterpret_cast<int*>(smem + SB_SEG_LIST) + 4;
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmap_q);
@@ -625,20 +721,32 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
   const uint32_t tmem_base = *tmem_slot;
   pdl_wait();
   pdl_trigger();
+  if (SEG) {         // every role walks the same list of query blocks whose id interval meets this key block's
+    if (warp == 2) {
+      const int nv = seg_visit_list(sg.rng_q + (size_t)b * nq, i0, nq, sg.rng_k[(size_t)b * nq + j], seg_list, lane);
+      if (lane == 0) seg_list[-1] = nv;
+    }
+    __syncthreads();
+    n_it = seg_list[-1];
+  }
   const uint32_t TM_S = tmem_base, TM_DP = tmem_base + 128, TM_DV = tmem_base + 256, TM_DK = tmem_base + 320,
                  TM_DQ = tmem_base + 384;
 
   if (warp == 0) {
     if (elect_one()) {
-      mbar_expect_tx(kv_full, 2 * TILE_BYTES);
-      tma_load_4d(smem + SB_K, &tmap_k, kv_full, 0, j * BKV, h, b);
-      tma_load_4d(smem + SB_V, &tmap_v, kv_full, 0, j * BKV, h, b);
+      if (!SEG || n_it > 0) {
+        mbar_expect_tx(kv_full, 2 * TILE_BYTES + (SEG ? BKV * 4 : 0));
+        tma_load_4d(smem + SB_K, &tmap_k, kv_full, 0, j * BKV, h, b);
+        tma_load_4d(smem + SB_V, &tmap_v, kv_full, 0, j * BKV, h, b);
+        if (SEG) bulk_load(seg_ids, sg.seg_k + b * sg.stride + j * BKV, BKV * 4, kv_full);
+      }
       for (int it = 0; it < n_it; ++it) {
         const int st = it & 1;
+        const int i = SEG ? seg_list[it] : i0 + it;
         mbar_wait(&q_empty[st], ((it >> 1) & 1) ^ 1);
         mbar_expect_tx(&q_full[st], 2 * TILE_BYTES);
-        tma_load_4d(smem + SB_Q + st * TILE_BYTES, &tmap_q, &q_full[st], 0, (i0 + it) * BQ, h, b);
-        tma_load_4d(smem + SB_DO + st * TILE_BYTES, &tmap_do, &q_full[st], 0, (i0 + it) * BQ, h, b);
+        tma_load_4d(smem + SB_Q + st * TILE_BYTES, &tmap_q, &q_full[st], 0, i * BQ, h, b);
+        tma_load_4d(smem + SB_DO + st * TILE_BYTES, &tmap_do, &q_full[st], 0, i * BQ, h, b);
       }
     }
   } else if (warp == 1) {
@@ -665,8 +773,10 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
                       idesc_s, k > 0 ? 1u : 0u);
         umma_commit(s_full);
       };
-      mbar_wait(kv_full, 0);
-      issue_sdp(0);
+      if (!SEG || n_it > 0) {
+        mbar_wait(kv_full, 0);
+        issue_sdp(0);
+      }
       for (int it = 0; it < n_it; ++it) {
         const int st = it & 1;
         mbar_wait(pds_full, it & 1);
@@ -699,7 +809,7 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
     const uint32_t lane_addr = uint32_t(quarter * 32) << 16;
     const float LOG2E = 1.4426950408889634f;
     for (int it = 0; it < n_it; ++it) {
-      const int i = i0 + it;
+      const int i = SEG ? seg_list[it] : i0 + it;
       const int q_global = i * BQ + row;
       const size_t stat_idx = ((size_t)b * p.H + h) * p.S + q_global;
       const float lse2 = p.lse[stat_idx] * LOG2E;
@@ -720,6 +830,24 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
       uint8_t* dsrow = smem + SB_DS + half * TILE_BYTES + row * 128;
       const bool diag = p.causal && (i == j);
       const int kv0 = j * BKV + half * 64;
+      uint32_t vis[2] = {~0u, ~0u};      // SEG: bit e of vis[c] = key kv0 + 32 c + e belongs to this row's document
+      if (SEG) {
+        const int my_seg = sg.seg_q[b * sg.stride + q_global];
+        const int2 kr = sg.rng_k[(size_t)b * nq + j];
+        if (!(kr.x == my_seg && kr.y == my_seg)) {
+          mbar_wait(kv_full, 0);           // (complete already: S was computed from this stage)
+          const int4* ids = reinterpret_cast<const int4*>(seg_ids + half * 64);
+#pragma unroll
+          for (int c = 0; c < 2; ++c) {
+            vis[c] = 0u;
+#pragma unroll
+            for (int g = 0; g < 8; ++g) {
+              const int4 id = ids[c * 8 + g];
+              vis[c] |= (uint32_t)((id.x == my_seg) | ((id.y == my_seg) << 1) | ((id.z == my_seg) << 2) | ((id.w == my_seg) << 3)) << (4 * g);
+            }
+          }
+        }
+      }
 #pragma unroll
       for (int c = 0; c < 2; ++c) {
         uint32_t pk[16], dk_[16];
@@ -734,6 +862,7 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
             const float xe = fmaf(sv_, p.scale_log2, -lse2);
             float pe = (POLY && u == 1) ? exp2_poly(xe) : exp2f(xe);
             if (diag && (kv0 + c * 32 + idx > q_global)) pe = 0.f;
+            if (SEG && !((vis[c] >> idx) & 1u)) pe = 0.f;
             pv[u] = pe;
             dsv[u] = pe * (dpv - delta);
           }
@@ -774,9 +903,14 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
     tc_fence_after();
     {
       uint32_t rv[32], rk[32];
-      tmem_ld_32x32(TM_DV + lane_addr + half * 32, rv);
-      tmem_ld_32x32(TM_DK + lane_addr + half * 32, rk);
-      tmem_ld_wait();
+      if (!SEG || n_it > 0) {
+        tmem_ld_32x32(TM_DV + lane_addr + half * 32, rv);
+        tmem_ld_32x32(TM_DK + lane_addr + half * 32, rk);
+        tmem_ld_wait();
+      } else {         // no query sees this key block: dK = dV = 0
+#pragma unroll
+        for (int i = 0; i < 32; ++i) rv[i] = rk[i] = 0u;
+      }
       const size_t off = (size_t)b * p.dstride_b + (size_t)(j * BKV + row) * p.dstride_s + (size_t)h * p.dstride_h + half * 32;
       uint4* dvp = reinterpret_cast<uint4*>(reinterpret_cast<__nv_bfloat16*>(p.dv) + off);
       uint4* dkp = reinterpret_cast<uint4*>(reinterpret_cast<__nv_bfloat16*>(p.dk) + off);
@@ -866,6 +1000,25 @@ EncodeTiledFn encode_fn() {
   return fn;
 }
 
+// Builds the AttnSeg of a masked call: checks the id layout and runs the [min, max] pre-pass into a persistent workspace.
+// Returns 0, or an error code.
+int seg_prepare(AttnSeg* sg, const void* seg_q, const void* seg_k, long long stride, int B, int S, cudaStream_t st) {
+  const int nblk = S / 128;
+  if (nblk > SEG_MAX_BLOCKS || stride < S || stride % 4 || ((uintptr_t)seg_q | (uintptr_t)seg_k) % 16) return -3;
+  static int2* ws = nullptr;
+  static size_t cap = 0;
+  const size_t need = (size_t)2 * B * nblk;
+  if (need > cap) {
+    if (ws) cudaFree(ws);
+    if (cudaMalloc(&ws, need * sizeof(int2)) != cudaSuccess) return -7;
+    cap = need;
+  }
+  sg->seg_q = (const int*)seg_q; sg->seg_k = (const int*)seg_k; sg->stride = stride;
+  sg->rng_q = ws; sg->rng_k = ws + (size_t)B * nblk;
+  const int warps = B * nblk;
+  return (int)tepd::launch(attn_seg_range_kernel, dim3((warps + 7) / 8, 2), dim3(256), 0, st, *sg, ws, ws + (size_t)B * nblk, B, nblk);
+}
+
 }  // namespace
 
 // 4-D map over a [B, S, H, D]-addressable bf16 tensor given element strides; box = {64, box_rows, 1, 1}.
@@ -884,9 +1037,10 @@ extern "C" int tepd_make_tmap_bshd(CUtensorMap* out, const void* ptr, int B, int
 }
 
 // q, k, v: bf16 pointers addressed as [B, S, H, D] with the given element strides (shared by q/k/v).
+// seg_q / seg_k: int32 document ids (row b at seg + b * seg_stride, 16-byte aligned), or null for the plain causal / full mask.
 extern "C" int tepd_attn_fwd(const void* q, const void* k, const void* v, void* o, void* lse, int B, int H, int S, int D,
                              float scale, int causal, long long stride_b, long long stride_s, long long stride_h,
-                             void* stream) {
+                             const void* seg_q, const void* seg_k, long long seg_stride, void* stream) {
   if (D != HD || S % 128 != 0) return -2;
   CUtensorMap tq, tk, tv;
   int rc = tepd_make_tmap_bshd(&tq, q, B, S, H, D, stride_b, stride_s, stride_h, BQ);
@@ -897,14 +1051,27 @@ extern "C" int tepd_attn_fwd(const void* q, const void* k, const void* v, void* 
   if (rc) return 300 + rc;
   static bool cfg = false;
   if (!cfg) {
-    cudaError_t e = cudaFuncSetAttribute(attn_fwd_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, FWD_SMEM);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_fwd_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, FWD_SMEM);
+    cudaError_t e = cudaFuncSetAttribute(attn_fwd_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, FWD_SMEM);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_fwd_kernel<1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, FWD_SMEM);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_fwd_kernel<0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, FWD_SEG_SMEM);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_fwd_kernel<1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, FWD_SEG_SMEM);
     if (e != cudaSuccess) return (int)e;
     cfg = true;
   }
   AttnFwdParams p;
   p.O = o; p.lse = (float*)lse; p.B = B; p.H = H; p.S = S; p.causal = causal;
   p.scale = scale; p.scale_log2 = scale * 1.4426950408889634f;
+  cudaStream_t cs = reinterpret_cast<cudaStream_t>(stream);
+  const int grid = (S / BQ) * B * H;
+  AttnSeg sg = {};
+  if (seg_q != nullptr || seg_k != nullptr) {   // document mask: always the default kernel (the two-tile variant has no mask)
+    if (seg_q == nullptr || seg_k == nullptr) return -3;
+    rc = seg_prepare(&sg, seg_q, seg_k, seg_stride, B, S, cs);
+    if (rc) return rc;
+    if (exp_poly_enabled())
+      return (int)tepd::launch(attn_fwd_kernel<1, 1>, dim3(grid), dim3(FWD_THREADS), FWD_SEG_SMEM, cs, tq, tk, tv, p, sg);
+    return (int)tepd::launch(attn_fwd_kernel<0, 1>, dim3(grid), dim3(FWD_THREADS), FWD_SEG_SMEM, cs, tq, tk, tv, p, sg);
+  }
   if (fwd2_enabled() && S % 256 == 0) {   // experimental two-tile kernel
     static bool cfg2 = false;
     if (!cfg2) {
@@ -915,10 +1082,9 @@ extern "C" int tepd_attn_fwd(const void* q, const void* k, const void* v, void* 
     return (int)tepd::launch(attn_fwd2_kernel, dim3((S / 256) * B * H), dim3(F2_THREADS), F2_SMEM, reinterpret_cast<cudaStream_t>(stream),
                              tq, tk, tv, p);
   }
-  int grid = (S / BQ) * B * H;
   if (exp_poly_enabled())
-    return (int)tepd::launch(attn_fwd_kernel<1>, dim3(grid), dim3(FWD_THREADS), FWD_SMEM, reinterpret_cast<cudaStream_t>(stream), tq, tk, tv, p);
-  return (int)tepd::launch(attn_fwd_kernel<0>, dim3(grid), dim3(FWD_THREADS), FWD_SMEM, reinterpret_cast<cudaStream_t>(stream), tq, tk, tv, p);
+    return (int)tepd::launch(attn_fwd_kernel<1, 0>, dim3(grid), dim3(FWD_THREADS), FWD_SMEM, cs, tq, tk, tv, p, sg);
+  return (int)tepd::launch(attn_fwd_kernel<0, 0>, dim3(grid), dim3(FWD_THREADS), FWD_SMEM, cs, tq, tk, tv, p, sg);
 }
 
 // (host) TEPDIST_ATTN_EXP_POLY=1 selects the POLY = 1 instantiations
@@ -926,7 +1092,8 @@ extern "C" int tepd_attn_fwd(const void* q, const void* k, const void* v, void* 
 extern "C" int tepd_attn_bwd(const void* dO, const void* q, const void* k, const void* v, const void* o, const void* lse,
                              void* dq_acc, void* dq, void* dk, void* dv, int B, int H, int S, int D, float scale,
                              int causal, long long stride_b, long long stride_s, long long stride_h, long long dstride_b,
-                             long long dstride_s, long long dstride_h, void* stream) {
+                             long long dstride_s, long long dstride_h, const void* seg_q, const void* seg_k,
+                             long long seg_stride, void* stream) {
   if (D != HD || S % 128 != 0) return -2;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   CUtensorMap tq, tk, tv, tdo;
@@ -967,8 +1134,10 @@ extern "C" int tepd_attn_bwd(const void* dO, const void* q, const void* k, const
   }
   static bool cfg = false;
   if (!cfg) {
-    cudaError_t e = cudaFuncSetAttribute(attn_bwd_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, BWD_SMEM);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_bwd_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, BWD_SMEM);
+    cudaError_t e = cudaFuncSetAttribute(attn_bwd_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, BWD_SMEM);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_bwd_kernel<1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, BWD_SMEM);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_bwd_kernel<0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, BWD_SEG_SMEM);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_bwd_kernel<1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, BWD_SEG_SMEM);
     if (e != cudaSuccess) return (int)e;
     cfg = true;
   }
@@ -976,9 +1145,19 @@ extern "C" int tepd_attn_bwd(const void* dO, const void* q, const void* k, const
   p.lse = (const float*)lse; p.delta = delta_buf; p.dq_acc = (float*)dq_acc; p.dk = dk; p.dv = dv;
   p.dstride_b = dstride_b; p.dstride_s = dstride_s; p.dstride_h = dstride_h;
   p.B = B; p.H = H; p.S = S; p.causal = causal; p.scale = scale; p.scale_log2 = scale * 1.4426950408889634f;
-  cudaError_t le = exp_poly_enabled()
-                       ? tepd::launch(attn_bwd_kernel<1>, dim3((S / BKV) * B * H), dim3(BWD_THREADS), BWD_SMEM, st, tq, tk, tv, tdo, p)
-                       : tepd::launch(attn_bwd_kernel<0>, dim3((S / BKV) * B * H), dim3(BWD_THREADS), BWD_SMEM, st, tq, tk, tv, tdo, p);
+  const dim3 grid((S / BKV) * B * H);
+  AttnSeg sg = {};
+  cudaError_t le;
+  if (seg_q != nullptr || seg_k != nullptr) {
+    if (seg_q == nullptr || seg_k == nullptr) return -3;
+    rc = seg_prepare(&sg, seg_q, seg_k, seg_stride, B, S, st);
+    if (rc) return rc;
+    le = exp_poly_enabled() ? tepd::launch(attn_bwd_kernel<1, 1>, grid, dim3(BWD_THREADS), BWD_SEG_SMEM, st, tq, tk, tv, tdo, p, sg)
+                            : tepd::launch(attn_bwd_kernel<0, 1>, grid, dim3(BWD_THREADS), BWD_SEG_SMEM, st, tq, tk, tv, tdo, p, sg);
+  } else {
+    le = exp_poly_enabled() ? tepd::launch(attn_bwd_kernel<1, 0>, grid, dim3(BWD_THREADS), BWD_SMEM, st, tq, tk, tv, tdo, p, sg)
+                            : tepd::launch(attn_bwd_kernel<0, 0>, grid, dim3(BWD_THREADS), BWD_SMEM, st, tq, tk, tv, tdo, p, sg);
+  }
   if (le != cudaSuccess) return (int)le;
   return (int)tepd::launch(attn_dq_cast_kernel, dim3(148 * 4), dim3(256), 0, st, (float*)dq_acc, (__nv_bfloat16*)dq, B, S, H,
                            dstride_b, dstride_s, dstride_h);

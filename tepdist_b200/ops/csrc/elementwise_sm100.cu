@@ -613,8 +613,10 @@ __global__ void __launch_bounds__(256) attn_merge_kernel(float* __restrict__ o_a
     }
     const float la = __ldg(lse_in + li);
     const float mx = fmaxf(la, lj);
-    const float nw = mx + __logf(__expf(la - mx) + __expf(lj - mx));
-    const float wa = __expf(la - nw), wj = __expf(lj - nw);
+    // both partials empty (document masking: no key of either block is visible to the row): stay at o = 0, lse = -inf
+    const bool empty = mx == -INFINITY;
+    const float nw = empty ? -INFINITY : mx + __logf(__expf(la - mx) + __expf(lj - mx));
+    const float wa = empty ? 0.f : __expf(la - nw), wj = empty ? 0.f : __expf(lj - nw);
     float4 a0 = oa[0], a1 = oa[1];
     a0.x = a0.x * wa + x[0] * wj; a0.y = a0.y * wa + x[1] * wj; a0.z = a0.z * wa + x[2] * wj; a0.w = a0.w * wa + x[3] * wj;
     a1.x = a1.x * wa + x[4] * wj; a1.y = a1.y * wa + x[5] * wj; a1.z = a1.z * wa + x[6] * wj; a1.w = a1.w * wa + x[7] * wj;

@@ -22,10 +22,12 @@ def plan_spmd(graph: Graph, num: int, strategy: str = "auto", options: Optional[
         strategy = "tp"
     if strategy in ("dp", "tp", "cp"):
         g = Graph.from_dict(graph.to_dict())
+        ids = _document_id_inputs(g.nodes)
         for n in g.nodes:
             if n.op == "input":
-                # "cp" (context parallel): every [batch, sequence, ...] sample input is cut along the SEQUENCE
-                dim = {"dp": 0, "tp": -1}.get(strategy, 1 if len(n.outputs[0].shape) >= 2 else -1)
+                # "cp" (context parallel): every [batch, sequence, ...] sample input is cut along the SEQUENCE, except attention's
+                # document ids, which every rank keeps whole (rules.cc AttentionRule)
+                dim = {"dp": 0, "tp": -1}.get(strategy, 1 if len(n.outputs[0].shape) >= 2 and n.id not in ids else -1)
                 n.attrs["sharding"] = {"0": {"dim": dim, "num": num}}
     cg = to_native(g)
     o = _C.SpmdOptions()
@@ -88,6 +90,22 @@ def plan_spmd(graph: Graph, num: int, strategy: str = "auto", options: Optional[
     return out, info
 
 
+def _document_id_inputs(nodes) -> set:
+    """Ids of the input nodes that feed attention its document ids (the optional last operand of attention / attention_bwd),
+    followed back through single-operand nodes (the slices an earlier mesh level inserted).  `nodes`: ir Nodes, or
+    (op, [input node ids]) pairs, indexed by node id."""
+    g = [(n.op, [v.node for v in n.inputs]) if hasattr(n, "op") else n for n in nodes]
+    out = set()
+    for op, ins in g:
+        k = {"attention": 1, "attention_bwd": 4}.get(op)
+        if k is not None and len(ins) > k:
+            i = ins[k]
+            while g[i][0] != "input" and len(g[i][1]) == 1:
+                i = g[i][1][0]
+            out.add(i)
+    return out
+
+
 def plan_spmd_mesh(graph: Graph, nums, kinds):
     """Multi-dimensional SPMD mesh (reference: one split ordinal per mesh dimension, dist_spec.h:130-227): plan and transform
     level 0 over nums[0] devices, then level 1 over nums[1] devices on the already sharded graph, ...  `kinds[i]` is
@@ -115,9 +133,11 @@ def plan_spmd_mesh(graph: Graph, nums, kinds):
         if kind == "cp":    # sequence split seeded on the sample inputs of THIS level, attention keeps it (K / V ring)
             o.context_parallel = True
             o.ignore_annotation = False
+            # ... except attention's document ids: every rank keeps them whole along the sequence (rules.cc AttentionRule)
+            ids = _document_id_inputs([(cg.node_op(i), [v[0] for v in cg.node_inputs(i)]) for i in range(cg.num_nodes())])
             for i in range(cg.num_nodes()):
                 if cg.node_op(i) == "input":
-                    cg.set_node_attr(i, "shard_dim", 1 if len(cg.node_outputs(i)[0][0]) >= 2 else -1)
+                    cg.set_node_attr(i, "shard_dim", 1 if len(cg.node_outputs(i)[0][0]) >= 2 and i not in ids else -1)
         plan = _C.plan_spmd_level(cg, o)
         if kind == "cp":
             for i in range(cg.num_nodes()):

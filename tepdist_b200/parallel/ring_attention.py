@@ -23,6 +23,11 @@ earlier rank j < r is two half-size unmasked products (both query chunks x the e
 others (the late query chunk x both chunks of j) -- n/2 block products per rank instead of up to n - 1/2.  CPU-validated
 (gloo, 2 and 4 ranks, against full attention); on GPUs it drives the same block kernels as the contiguous ring but has not
 run there yet, hence opt-in.
+
+Document masking (`segments`, int32 [B, S]): the ids stay whole along the sequence on every rank of the ring (the planner keeps
+them unsplit there), so a rank slices the query ids of its own block and the key ids of each visiting block locally and the ring
+moves no extra bytes.  A (query block, key block) product whose id intervals do not overlap in any sequence of the batch is
+skipped (`blocks_skipped`); a computed block whose rows see none of its keys contributes o = 0, lse = -inf to the merge.
 """
 from __future__ import annotations
 
@@ -45,6 +50,31 @@ class RingAttention:
         self.bytes_moved = 0
         self.zigzag = (os.environ.get("TEPDIST_CP_ZIGZAG") == "1") if zigzag is None else bool(zigzag)
         self.block_products = 0.0            # work done by this rank, in units of one full L x L block product (diagnostic)
+        self.blocks_skipped = 0.0            # block products left out because their document ids cannot meet (same units)
+
+    # ---------------------------------------------------------------- document ids
+    class _Seg:
+        """The document ids [B, S] of the whole sequence cut into `chunks` equal pieces; `meets(a, b)` tells whether any query
+        of piece a can see a key of piece b (one host read of the per-piece [min, max] per call: the ring runs eagerly)."""
+
+        def __init__(self, seg: torch.Tensor, chunks: int):
+            B, S = seg.shape
+            self.seg, self.size = seg.to(torch.int32), S // chunks
+            v = self.seg.reshape(B, chunks, self.size)
+            self.mn, self.mx = v.amin(2).cpu(), v.amax(2).cpu()
+
+        def ids(self, *pieces: int) -> torch.Tensor:
+            return torch.cat([self.seg[:, c * self.size:(c + 1) * self.size] for c in pieces], 1).contiguous()
+
+        def meets(self, a: int, b: int) -> bool:
+            return bool(((self.mn[:, a] <= self.mx[:, b]) & (self.mn[:, b] <= self.mx[:, a])).any())
+
+    def _segments(self, segments: Optional[torch.Tensor], L: int, zigzag: bool):
+        if segments is None:
+            return None
+        chunks = 2 * self.n if zigzag else self.n
+        assert segments.shape[1] == self.n * L, ("document ids must cover the whole sequence", tuple(segments.shape), L)
+        return self._Seg(segments, chunks)
 
     # ---------------------------------------------------------------- ring plumbing
     def _exchange(self, send: torch.Tensor, recv: torch.Tensor):
@@ -72,13 +102,17 @@ class RingAttention:
         return w
 
     # ---------------------------------------------------------------- forward
-    def forward(self, q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, causal: bool = True, scale: Optional[float] = None
-                ) -> Tuple[torch.Tensor, torch.Tensor]:
+    def forward(self, q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, causal: bool = True, scale: Optional[float] = None,
+                segments: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+        """`segments`: optional document ids [B, n L] of the WHOLE sequence (module docstring)."""
         B, L, H, D = q.shape
         scale = 1.0 / math.sqrt(D) if scale is None else scale
         n, r = self.n, self.index
-        if self._use_zigzag(q, causal):
-            return self._forward_zigzag(q, k, v, scale)
+        zz = self._use_zigzag(q, causal)
+        sg = self._segments(segments, L, zz)
+        if zz:
+            return self._forward_zigzag(q, k, v, scale, sg)
+        sq = sg.ids(r) if sg is not None else None
         o_acc = torch.empty(B, L, H, D, dtype=torch.float32, device=q.device)
         lse_acc, lse_nxt = (torch.empty(B, H, L, dtype=torch.float32, device=q.device) for _ in range(2))
         first = True
@@ -88,13 +122,16 @@ class RingAttention:
         for t in range(n):
             j = (r - t) % n
             reqs = self._exchange(cur, nxt) if t < n - 1 else []
-            if not (causal and j > r):
+            if not (causal and j > r) and sg is not None and not sg.meets(r, j):
+                self.blocks_skipped += 1.0
+            elif not (causal and j > r):
                 self.block_products += 0.5 if (causal and t == 0) else 1.0
+                sk = sg.ids(j) if sg is not None else None
                 if t == 0:
-                    o_j, lse_j = attention_fwd(q, k, v, scale, causal)
+                    o_j, lse_j = attention_fwd(q, k, v, scale, causal, seg_q=sq, seg_k=sk)
                 else:
                     work[:, :, :, 1:].copy_(cur)
-                    o_j, lse_j = attention_fwd(work[:, :, :, 0], work[:, :, :, 1], work[:, :, :, 2], scale, False)
+                    o_j, lse_j = attention_fwd(work[:, :, :, 0], work[:, :, :, 1], work[:, :, :, 2], scale, False, seg_q=sq, seg_k=sk)
                 attn_merge_(o_acc, lse_acc, lse_nxt, o_j.contiguous(), lse_j.contiguous(), first)   # one kernel per block
                 lse_acc, lse_nxt, first = lse_nxt, lse_acc, False
             self._wait(reqs)
@@ -103,15 +140,19 @@ class RingAttention:
 
     # ---------------------------------------------------------------- backward
     def backward(self, do: torch.Tensor, q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, o: torch.Tensor, lse: torch.Tensor,
-                 causal: bool = True, scale: Optional[float] = None, dqkv_out: Optional[torch.Tensor] = None):
+                 causal: bool = True, scale: Optional[float] = None, dqkv_out: Optional[torch.Tensor] = None,
+                 segments: Optional[torch.Tensor] = None):
         """Returns (dq, dk, dv) as views of `dqkv_out` [B,L,H,3,D]."""
         B, L, H, D = q.shape
         scale = 1.0 / math.sqrt(D) if scale is None else scale
         n, r = self.n, self.index
         if dqkv_out is None:
             dqkv_out = torch.empty(B, L, H, 3, D, dtype=q.dtype, device=q.device)
-        if self._use_zigzag(q, causal):
-            return self._backward_zigzag(do, q, k, v, o, lse, scale, dqkv_out)
+        zz = self._use_zigzag(q, causal)
+        sg = self._segments(segments, L, zz)
+        if zz:
+            return self._backward_zigzag(do, q, k, v, o, lse, scale, dqkv_out, sg)
+        sq = sg.ids(r) if sg is not None else None
         do, o, lse = do.contiguous(), o.contiguous(), lse.contiguous()
         cur = torch.stack((k, v), 3).contiguous()
         nxt = torch.empty_like(cur)
@@ -123,13 +164,17 @@ class RingAttention:
         for t in range(n):
             j = (r - t) % n
             reqs = self._exchange(cur, nxt) if t < n - 1 else []
-            if not (causal and j > r):
+            if not (causal and j > r) and sg is not None and not sg.meets(r, j):
+                self.blocks_skipped += 1.0
+            elif not (causal and j > r):
                 self.block_products += 0.5 if (causal and t == 0) else 1.0
+                sk = sg.ids(j) if sg is not None else None
                 if t == 0:
-                    attention_bwd(do, q, k, v, o, lse, scale, causal, dqkv_out=part)
+                    attention_bwd(do, q, k, v, o, lse, scale, causal, dqkv_out=part, seg_q=sq, seg_k=sk)
                 else:
                     work[:, :, :, 1:].copy_(cur)
-                    attention_bwd(do, work[:, :, :, 0], work[:, :, :, 1], work[:, :, :, 2], o, lse, scale, False, dqkv_out=part)
+                    attention_bwd(do, work[:, :, :, 0], work[:, :, :, 1], work[:, :, :, 2], o, lse, scale, False, dqkv_out=part,
+                                  seg_q=sq, seg_k=sk)
                 attn_ring_accum_(dq_acc, acc, part)
             self._wait(reqs)
             # the accumulator follows its block: after the last step it is one hop from home
@@ -199,12 +244,26 @@ class RingAttention:
         j = (self.index - t) % self.n
         return ((0, 0), (1, 0)) if j < self.index else ((1, 0), (1, 1))
 
-    def _forward_zigzag(self, q, k, v, scale):
+    def _zz_chunks(self, rank: int) -> Tuple[int, int]:
+        """Global chunks (of 2n) that `rank` holds in the zig-zag layout: (early, late)."""
+        return rank, 2 * self.n - 1 - rank
+
+    def _zz_pair_ids(self, sg, t: int, qh: int, kh: int):
+        """(query ids, key ids) of product (qh, kh) at ring step t, or None when the product is skipped."""
+        if sg is None:
+            return None, None
+        cq, ck = self._zz_chunks(self.index)[qh], self._zz_chunks((self.index - t) % self.n)[kh]
+        if not sg.meets(cq, ck):
+            return None
+        return sg.ids(cq), sg.ids(ck)
+
+    def _forward_zigzag(self, q, k, v, scale, sg=None):
         B, L, H, D = q.shape
         n, l, dev = self.n, L // 2, q.device
         qkv = self._permute(torch.stack((q, k, v), 3), True)                   # [B,L,H,3,D] in the zig-zag layout
         qz, kz, vz = qkv[:, :, :, 0], qkv[:, :, :, 1], qkv[:, :, :, 2]
-        o0, lse0 = attention_fwd(qz, kz, vz, scale, True)                      # local step: causal over [early; late]
+        sz = sg.ids(*self._zz_chunks(self.index)) if sg is not None else None
+        o0, lse0 = attention_fwd(qz, kz, vz, scale, True, seg_q=sz, seg_k=sz)  # local step: causal over [early; late]
         self.block_products += 0.5
         o_acc = torch.empty(2, B, l, H, D, dtype=torch.float32, device=dev)
         lse_a = [torch.empty(B, H, l, dtype=torch.float32, device=dev) for _ in range(2)]
@@ -224,8 +283,13 @@ class RingAttention:
             cur, nxt = nxt, cur
             reqs = self._exchange(cur, nxt) if t < n - 1 else []
             for qh, kh in self._pairs(t):
+                ids = self._zz_pair_ids(sg, t, qh, kh)
+                if ids is None:
+                    self.blocks_skipped += 0.25
+                    continue
                 work[qh][:, :, :, 1:].copy_(cur[kh])
-                o_j, lse_j = attention_fwd(work[qh][:, :, :, 0], work[qh][:, :, :, 1], work[qh][:, :, :, 2], scale, False)
+                o_j, lse_j = attention_fwd(work[qh][:, :, :, 0], work[qh][:, :, :, 1], work[qh][:, :, :, 2], scale, False,
+                                           seg_q=ids[0], seg_k=ids[1])
                 attn_merge_(o_acc[qh], lse_a[qh], lse_b[qh], o_j.contiguous(), lse_j.contiguous(), False)
                 lse_a[qh], lse_b[qh] = lse_b[qh], lse_a[qh]
                 self.block_products += 0.25
@@ -236,7 +300,7 @@ class RingAttention:
         # which works in the zig-zag layout: it stays there
         return self._permute(o, False), lse
 
-    def _backward_zigzag(self, do, q, k, v, o, lse, scale, dqkv_out):
+    def _backward_zigzag(self, do, q, k, v, o, lse, scale, dqkv_out, sg=None):
         B, L, H, D = q.shape
         n, l, dev = self.n, L // 2, q.device
         qkv = self._permute(torch.stack((q, k, v), 3), True)
@@ -245,7 +309,8 @@ class RingAttention:
         doz, oz = go[:, :, :, 0].contiguous(), go[:, :, :, 1].contiguous()
         lse = lse.contiguous()
         part = torch.empty(B, L, H, 3, D, dtype=q.dtype, device=dev)
-        attention_bwd(doz, qz, kz, vz, oz, lse, scale, True, dqkv_out=part)    # local step
+        sz = sg.ids(*self._zz_chunks(self.index)) if sg is not None else None
+        attention_bwd(doz, qz, kz, vz, oz, lse, scale, True, dqkv_out=part, seg_q=sz, seg_k=sz)    # local step
         self.block_products += 0.5
         ph = self._halves(part)                                                # [2,B,l,H,3,D]
         dq_acc = ph[:, :, :, :, 0].float().contiguous()                        # [2,B,l,H,D]
@@ -269,9 +334,13 @@ class RingAttention:
             cur, nxt = nxt, cur
             reqs = self._exchange(cur, nxt) if t < n - 1 else []
             for qh, kh in self._pairs(t):
+                ids = self._zz_pair_ids(sg, t, qh, kh)
+                if ids is None:
+                    self.blocks_skipped += 0.25
+                    continue
                 work[qh][:, :, :, 1:].copy_(cur[kh])
                 attention_bwd(doh[qh], work[qh][:, :, :, 0], work[qh][:, :, :, 1], work[qh][:, :, :, 2], oh[qh], lh[qh], scale, False,
-                              dqkv_out=small)
+                              dqkv_out=small, seg_q=ids[0], seg_k=ids[1])
                 attn_ring_accum_(dq_acc[qh], acc[kh], small)
                 self.block_products += 0.25
         gz = torch.empty(B, L, H, 3, D, dtype=q.dtype, device=dev)

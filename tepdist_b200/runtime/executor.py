@@ -1371,18 +1371,21 @@ class Executor:
             return [ops.gelu_bwd(ins[0], ins[1])]
         if op == "attention":
             qkv = ins[0]
+            seg = ins[1] if len(ins) > 1 else None     # document ids: whole along the sequence (rules.cc AttentionRule)
             B, S, C3 = qkv.shape
             H = a["heads"]
             D = C3 // 3 // H
             q5 = qkv.view(B, S, H, 3, D)  # heads-major: a last-dim split is a split over heads
             ring = self._ring(n)
             if ring is not None:    # context parallel: S is this rank's block of the sequence, K / V blocks ride the ring
-                o, lse = ring.forward(q5[:, :, :, 0], q5[:, :, :, 1], q5[:, :, :, 2], causal=a.get("causal", True))
+                o, lse = ring.forward(q5[:, :, :, 0], q5[:, :, :, 1], q5[:, :, :, 2], causal=a.get("causal", True), segments=seg)
                 return [o.reshape(B, S, H * D), lse]
-            o, lse = ops.attention_fwd(q5[:, :, :, 0], q5[:, :, :, 1], q5[:, :, :, 2], causal=a.get("causal", True))
+            o, lse = ops.attention_fwd(q5[:, :, :, 0], q5[:, :, :, 1], q5[:, :, :, 2], causal=a.get("causal", True),
+                                       seg_q=seg, seg_k=seg)
             return [o.view(B, S, H * D), lse]
         if op == "attention_bwd":
-            do, qkv, o, lse = ins
+            do, qkv, o, lse = ins[:4]
+            seg = ins[4] if len(ins) > 4 else None
             B, S, C3 = qkv.shape
             H = a["heads"]
             D = C3 // 3 // H
@@ -1391,10 +1394,10 @@ class Executor:
             ring = self._ring(n)
             if ring is not None:
                 ring.backward(do.reshape(B, S, H, D), q5[:, :, :, 0], q5[:, :, :, 1], q5[:, :, :, 2], o.reshape(B, S, H, D), lse,
-                              causal=a.get("causal", True), dqkv_out=dqkv)
+                              causal=a.get("causal", True), dqkv_out=dqkv, segments=seg)
                 return [dqkv.view(B, S, C3)]
             ops.attention_bwd(do.reshape(B, S, H, D), q5[:, :, :, 0], q5[:, :, :, 1], q5[:, :, :, 2], o.reshape(B, S, H, D),
-                              lse, causal=a.get("causal", True), dqkv_out=dqkv)
+                              lse, causal=a.get("causal", True), dqkv_out=dqkv, seg_q=seg, seg_k=seg)
             return [dqkv.view(B, S, C3)]
         if op == "softmax_xent":
             logits, labels = ins
